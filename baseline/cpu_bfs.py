@@ -17,7 +17,7 @@ ROOT = os.path.dirname(HERE)
 OUT = os.path.join(ROOT, "build", "cpu_baseline")
 
 
-def build(model: str) -> str:
+def build(model: str, out_dir: str = OUT) -> str:
     hdr = os.path.join(ROOT, "build", "models", model, "model.h")
     src = os.path.join(HERE, "cpu_bfs.cpp")
     if not os.path.exists(hdr):
@@ -31,16 +31,16 @@ def build(model: str) -> str:
     except OSError:
         pass
     tag = hashlib.sha256(open(hdr, "rb").read() + open(src, "rb").read() + cpu).hexdigest()[:12]
-    os.makedirs(OUT, exist_ok=True)
-    so = os.path.join(OUT, f"cpu_{model}_{tag}.so")
+    os.makedirs(out_dir, exist_ok=True)
+    so = os.path.join(out_dir, f"cpu_{model}_{tag}.so")
     if not os.path.exists(so):
         subprocess.check_call(["g++", "-O3", "-march=native", "-std=c++20", "-pthread", "-shared", "-fPIC",
                                f'-DKMC_MODEL_HEADER="{hdr}"', src, "-o", so])
     return so
 
 
-def run(model: str, threads: int = 0, table_log2: int = 24, stop_after_states: int = 0) -> dict:
-    lib = ctypes.CDLL(build(model))
+def run(model: str, threads: int = 0, table_log2: int = 24, stop_after_states: int = 0, out_dir: str = OUT) -> dict:
+    lib = ctypes.CDLL(build(model, out_dir))
     lib.kmc_cpu_bfs.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_uint64]
     st = np.zeros(320, dtype=np.uint64)
     rc = lib.kmc_cpu_bfs(st.ctypes.data, threads, table_log2, stop_after_states)

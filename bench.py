@@ -1,6 +1,6 @@
 """bench.py -- distinct states/sec of the BFS frontier-expansion path on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--model NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--model NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one complete explicit-state BFS (Init -> empty frontier) of the headline model:
@@ -23,28 +23,90 @@ per-level widths) is compared with the committed golden before a number is print
                TLC itself cannot run here, no JVM).  Oracle B stays what it is: the checker.
 
 --impl reference times that CPU path alone (rank 0 only).
+
+--dump-outputs DIR writes what the last timed step computed (single GPU), for comparing two builds:
+  counts.npy         float64 [distinct, generated, depth, queue, deadlocks, complete]
+  levels.npy         float64 per-level widths (distinct states first reached at each BFS level)
+  states_sample.npy  float64 [rows, 2*words]: the reachable states whose salted hash falls in a fixed residue
+                     class (about 2^18 of them), each 64-bit word split into its high and low 32 bits, rows
+                     sorted -- a sample chosen by content, so it does not depend on the order of the state store
+Nothing is written to the source tree: run-time builds (the cold-start nvcc output, the CPU arm's library) go to a
+temporary directory removed at exit.
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
+import shutil
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 DEFAULT_MODEL = "kip320_3x4_r4e3"
 METRIC = "distinct states/sec"
+SAMPLE_SALT = 0x5EED_0F_C0FFEE          # fixed seed of the state sample written by --dump-outputs
+SAMPLE_ROWS_LOG2 = 18                  # about 2^18 sampled states: 2^18 rows * 2 words * 2 halves * 8 B = 8 MB for W = 2
+
+_SCRATCH = None
+
+
+def scratch_dir() -> str:
+    """A private temporary directory for what the benchmark compiles at run time; the tree may be read-only."""
+    global _SCRATCH
+    if _SCRATCH is None:
+        _SCRATCH = tempfile.mkdtemp(prefix="kspec-bench-")
+        atexit.register(shutil.rmtree, _SCRATCH, True)
+    return _SCRATCH
 
 
 def load_json(path):
     with open(path) as f:
         return json.load(f)
+
+
+def _mix64(x: np.ndarray) -> np.ndarray:
+    """splitmix64 finaliser on uint64 arrays (wrapping arithmetic)."""
+    x = x ^ (x >> np.uint64(30))
+    x = x * np.uint64(0xBF58476D1CE4E5B9)
+    x = x ^ (x >> np.uint64(27))
+    x = x * np.uint64(0x94D049BB133111EB)
+    return x ^ (x >> np.uint64(31))
+
+
+def sample_states(ck, distinct: int, chunk_rows: int = 1 << 24) -> np.ndarray:
+    """The reachable states whose salted content hash is 0 modulo max(1, distinct >> SAMPLE_ROWS_LOG2), sorted;
+    returned as float64 with every uint64 word split into (high 32 bits, low 32 bits), which float64 holds exactly."""
+    modulus = np.uint64(max(1, distinct >> SAMPLE_ROWS_LOG2))
+    picked = []
+    for first in range(0, distinct, chunk_rows):
+        rows = ck.copy_states(first, min(chunk_rows, distinct - first))
+        h = np.full(len(rows), SAMPLE_SALT, dtype=np.uint64)
+        for k in range(rows.shape[1]):
+            h = _mix64(h ^ rows[:, k])
+        picked.append(rows[h % modulus == 0])
+    rows = np.concatenate(picked) if picked else np.zeros((0, ck.words), dtype=np.uint64)
+    rows = rows[np.lexsort(rows.T[::-1])] if len(rows) else rows
+    halves = np.stack([rows >> np.uint64(32), rows & np.uint64(0xFFFFFFFF)], axis=2).reshape(len(rows), -1)
+    return halves.astype(np.float64)
+
+
+def dump_outputs(out_dir: str, ck, res) -> None:
+    """Writes the last timed step's result (see the module docstring) as float64 .npy files."""
+    os.makedirs(out_dir, exist_ok=True)
+    counts = [res.distinct, res.generated, res.depth, res.queue, res.deadlocks, int(res.complete)]
+    np.save(os.path.join(out_dir, "counts.npy"), np.array(counts, dtype=np.float64))
+    np.save(os.path.join(out_dir, "levels.npy"), np.array(res.levels, dtype=np.float64))
+    np.save(os.path.join(out_dir, "states_sample.npy"), sample_states(ck, res.distinct))
 
 
 def measured_peaks():
@@ -147,13 +209,14 @@ def cpu_run(model: str, threads: int = 0, budget_s: float = 25.0, table_log2: in
         table_log2 = 20
         while (1 << table_log2) < 2.5 * max(total, 1 << 18):
             table_log2 += 1
-    probe = cpu_bfs.run(model, threads, min(table_log2, 26), stop_after_states=2_000_000)
+    probe = cpu_bfs.run(model, threads, min(table_log2, 26), stop_after_states=2_000_000, out_dir=scratch_dir())
     rate = probe["distinct"] / max(probe["seconds"], 1e-9)
     full = bool(total) and (probe["complete"] or total / rate <= budget_s)
     if probe["complete"]:
         r = probe
     else:
-        r = cpu_bfs.run(model, threads, table_log2, stop_after_states=0 if full else int(rate * budget_s))
+        r = cpu_bfs.run(model, threads, table_log2, stop_after_states=0 if full else int(rate * budget_s),
+                        out_dir=scratch_dir())
     if r["fail"]:
         raise SystemExit(f"cpu baseline failed on {model}: code {r['fail']}")
     if r["complete"] and g:
@@ -177,7 +240,7 @@ def cpu_scaling(model: str):
     for t in (1, 16):
         if t > (os.cpu_count() or 1):
             continue
-        r = cpu_bfs.run(model, t, 25, stop_after_states=1_500_000 * t)
+        r = cpu_bfs.run(model, t, 25, stop_after_states=1_500_000 * t, out_dir=scratch_dir())
         out[str(t)] = round(r["distinct"] / max(r["seconds"], 1e-9))
     return out
 
@@ -234,9 +297,7 @@ def cold_start(model: str, opts: dict):
     from kafka_specification_b200 import build as B
     from kafka_specification_b200.runtime import Checker
     meta = load_json(os.path.join(B.model_dir(model), "model.json"))
-    out = os.path.join(ROOT, "build", "cold")
-    os.makedirs(out, exist_ok=True)
-    so = os.path.join(out, f"libkmc_{model}.cold.so")
+    so = os.path.join(scratch_dir(), f"libkmc_{model}.cold.so")
     t0 = time.perf_counter()
     B.compile_model_to(model, so)
     t1 = time.perf_counter()
@@ -289,6 +350,8 @@ def run_single(args):
     torch.cuda.synchronize()
     bracket_ms = 1000.0 * (time.perf_counter() - t_bracket)
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ck, res)
     parity = check_result(args.model, res.distinct, res.generated, res.depth, res.levels, res.deadlocks)
     if res.violation is not None or not res.complete:
         raise SystemExit(f"bench: unexpected verdict {res.violation}")
@@ -514,7 +577,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-cold", action="store_true", help="skip the cold-start (nvcc + first run) measurement")
     ap.add_argument("--no-p2p", action="store_true", help="multi-GPU: NCCL all-to-all exchange instead of the fused peer-memory path")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="single GPU: write the last timed step's result to DIR/*.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     # Sizing is configuration (like TLC's -fpmem), not derived from the answer: 2^30 set slots and room for 2^29
@@ -524,6 +591,8 @@ def main():
         args.table_log2 = 30 if world == 1 else 29
     if not args.max_states:
         args.max_states = (1 << 29) if world == 1 else (1 << 28)
+    if args.dump_outputs and (args.impl == "reference" or world > 1):
+        ap.error("--dump-outputs is supported for the single-GPU run of --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     if world > 1:

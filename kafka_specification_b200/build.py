@@ -3,16 +3,18 @@
     python -m kafka_specification_b200.build --all            # every model in models/MODELS.json
     python -m kafka_specification_b200.build Kip320 models/Kip320.cfg --name kip320
 
-Artifacts go to ``build/`` (git-ignored, shipped to the GPU box by gpurun):
+Artifacts go to ``build/`` (git-ignored):
 
     build/libkspecmc.so                 the C-ABI dispatcher (include/kspecmc.h)
     build/models/<name>/model.h         the lowered switch table
     build/models/<name>/model.json      layout / actions / invariants (for trace printing)
     build/models/<name>/libkmc_<name>.so
 
-The ``.tla`` sources are read from the reference checkout (``KSPEC_TLA_PATH`` or /root/reference)
-and from ``models/``; they are not copied into this repository.  On a machine without the
-reference (the GPU box) the prebuilt artifacts are used as they are.
+The ``.tla`` sources are read from the kafka-specification checkout (``KSPEC_TLA_PATH``, or the
+default location in ``tla_search_dirs``) and from ``models/``; they are not copied into this
+repository.  A build that can read them also saves each lowered model.h / model.json under
+``oracle/_ref/models/<name>/`` (git-ignored: it is derived data of the specification); a build on a
+machine without the specification (a GPU machine given that directory) compiles those saved headers.
 """
 from __future__ import annotations
 
@@ -29,6 +31,9 @@ BUILD = os.path.join(ROOT, "build")
 CSRC = os.path.join(ROOT, "kafka_specification_b200", "csrc")
 INCLUDE = os.path.join(ROOT, "include")
 MODELS_DIR = os.path.join(ROOT, "models")
+SPECS_DIR = os.path.join(ROOT, "tests", "specs")
+SAVED_MODELS = os.path.join(ROOT, "oracle", "_ref", "models")
+LOWERED_FILES = ("model.h", "model.json")
 
 NVCC_ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 
@@ -40,6 +45,11 @@ def tla_search_dirs() -> list[str]:
         dirs += env.split(os.pathsep)
     dirs += ["/root/reference", MODELS_DIR, os.path.join(ROOT, "tests", "specs")]
     return [d for d in dirs if os.path.isdir(d)]
+
+
+def specification_reachable() -> bool:
+    """True when a .tla search directory outside this repository (the kafka-specification checkout) exists."""
+    return any(d not in (MODELS_DIR, SPECS_DIR) for d in tla_search_dirs())
 
 
 def nvcc_path() -> str:
@@ -156,13 +166,27 @@ def compile_model_to(name: str, out_so: str) -> str:
     return out_so
 
 
-def build_model(module: str, cfg_path: str, name: str, force: bool = False) -> str:
-    """Lower (when the .tla sources are reachable) and compile; returns the library path."""
-    have_sources = any(os.path.exists(os.path.join(d, module + ".tla")) for d in tla_search_dirs())
-    if have_sources:
+def prepare_model(module: str, cfg_path: str, name: str) -> None:
+    """Puts build/models/<name>/model.h and model.json in place.  With the specification reachable the model is
+    lowered and saved under oracle/_ref/models/<name>/; without it the saved copy is used when there is one, else
+    the model is lowered from this repository's own modules (a module that is not there raises ModuleError)."""
+    saved = os.path.join(SAVED_MODELS, name)
+    if specification_reachable():
         lower_to_dir(module, cfg_path, name)
-    elif not os.path.exists(os.path.join(model_dir(name), "model.h")):
-        raise RuntimeError(f"{module}.tla is not reachable and build/models/{name}/model.h was not prebuilt")
+        os.makedirs(saved, exist_ok=True)
+        for f in LOWERED_FILES:
+            shutil.copyfile(os.path.join(model_dir(name), f), os.path.join(saved, f))
+    elif all(os.path.exists(os.path.join(saved, f)) for f in LOWERED_FILES):
+        os.makedirs(model_dir(name), exist_ok=True)
+        for f in LOWERED_FILES:
+            shutil.copyfile(os.path.join(saved, f), os.path.join(model_dir(name), f))
+    else:
+        lower_to_dir(module, cfg_path, name)
+
+
+def build_model(module: str, cfg_path: str, name: str, force: bool = False) -> str:
+    """Lower (or take the saved lowering, see prepare_model) and compile; returns the library path."""
+    prepare_model(module, cfg_path, name)
     return compile_model(name, force=force)
 
 
@@ -179,12 +203,7 @@ def build_all(force: bool = False, only: list[str] | None = None, verbose: bool 
     for name, spec in registry().items():
         if only and name not in only:
             continue
-        module, cfg_path = spec["module"], os.path.join(ROOT, spec["cfg"])
-        have_sources = any(os.path.exists(os.path.join(d, module + ".tla")) for d in tla_search_dirs())
-        if have_sources:
-            lower_to_dir(module, cfg_path, name)
-        elif not os.path.exists(os.path.join(model_dir(name), "model.h")):
-            raise RuntimeError(f"{module}.tla is not reachable and build/models/{name}/model.h was not prebuilt")
+        prepare_model(spec["module"], os.path.join(ROOT, spec["cfg"]), name)
         todo.append(name)
     jobs = jobs or min(8, os.cpu_count() or 1)
 

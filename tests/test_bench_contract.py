@@ -44,7 +44,7 @@ def test_single_gpu_line_has_the_contract_keys(monkeypatch, capsys, goldens):
     monkeypatch.setattr(runtime, "Checker", FakeChecker)
     monkeypatch.setattr(bench, "cold_start", lambda model, opts: {"seconds": 1.0, "stub": True})
     args = types.SimpleNamespace(model="kip320_small", warmup=1, steps=2, table_log2=24, max_states=1 << 23,
-                                 no_cpu_baseline=False, no_cold=False)
+                                 no_cpu_baseline=False, no_cold=False, dump_outputs=None)
     assert bench.run_single(args) == 0
     line = json.loads([l for l in capsys.readouterr().out.splitlines() if l.startswith("{")][-1])
     for k in ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling",
@@ -89,11 +89,64 @@ def test_auxiliary_leg_failure_does_not_cost_the_line(monkeypatch, capsys, golde
     monkeypatch.setattr(bench, "cold_start", boom)
     monkeypatch.setattr(bench, "cpu_run", boom)
     args = types.SimpleNamespace(model="kip320_small", warmup=1, steps=1, table_log2=24, max_states=1 << 23,
-                                 no_cpu_baseline=False, no_cold=False)
+                                 no_cpu_baseline=False, no_cold=False, dump_outputs=None)
     assert bench.run_single(args) == 0
     line = json.loads([l for l in capsys.readouterr().out.splitlines() if l.startswith("{")][-1])
     assert line["value"] > 0 and "nvcc exploded" in line["e2e_cold"]["error"]
     assert line["cpu_baseline"]["value"] is None and "failed" in line["cpu_baseline"]["sample"]
+
+
+def test_dump_outputs_is_the_last_step_and_independent_of_store_order(monkeypatch, capsys, goldens, tmp_path):
+    """--dump-outputs writes float64 counts, level widths and a state sample chosen by content: two state stores
+    holding the same set in different orders give identical files, and every sampled row is an exact stored state."""
+    import numpy as np
+    import torch
+    import bench
+    from kafka_specification_b200 import runtime
+    g = goldens["kip320_small"]
+    store = np.random.default_rng(3).integers(0, np.iinfo(np.uint64).max, size=(g["distinct"], 2),
+                                              dtype=np.uint64, endpoint=True)
+    runs = []
+
+    class FakeChecker:
+        def __init__(self, model, **opts):
+            self.words = 2
+            self.info = types.SimpleNamespace(exact=1, num_init=1)
+            self.store = store[np.random.default_rng(len(runs)).permutation(len(store))]
+            self.steps = 0
+
+        def run(self):
+            self.steps += 1
+            r = _FakeResult(g, self.words)
+            r.queue = self.steps                  # tells the steps apart: the dump must be the last one's
+            return r
+
+        def copy_states(self, first, count):
+            return self.store[first:first + count].copy()
+
+        def close(self):
+            pass
+
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: True)
+    monkeypatch.setattr(torch.cuda, "synchronize", lambda *a, **k: None)
+    monkeypatch.setattr(runtime, "Checker", FakeChecker)
+    for i in range(2):
+        out = tmp_path / str(i)
+        args = types.SimpleNamespace(model="kip320_small", warmup=1, steps=3, table_log2=24, max_states=1 << 23,
+                                     no_cpu_baseline=True, no_cold=True, dump_outputs=str(out))
+        assert bench.run_single(args) == 0
+        runs.append({f: np.load(out / f) for f in ("counts.npy", "levels.npy", "states_sample.npy")})
+    a, b = runs
+    assert all(v.dtype == np.float64 for v in a.values())
+    # queue = 4: the 4th call of run() (1 warm-up + 3 timed steps)
+    assert a["counts.npy"].tolist() == [g["distinct"], g["generated"], g["depth"], 4, g["deadlocks"], 1]
+    assert a["levels.npy"].tolist() == g["levels"]
+    s = a["states_sample.npy"]
+    assert s.shape[1] == 4 and 1 << 16 < len(s) < 1 << 20 and sum(v.nbytes for v in a.values()) < 64 << 20
+    assert all(np.array_equal(a[k], b[k]) for k in a)
+    words = s.astype(np.uint64).reshape(len(s), 2, 2)
+    rows = (words[:, :, 0] << np.uint64(32)) | words[:, :, 1]
+    assert set(map(tuple, rows.tolist())) <= set(map(tuple, store.tolist()))
 
 
 def _run_sharded_worker(model, inject, port):
